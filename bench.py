@@ -9,6 +9,7 @@ iterations, max over ranks; the e2e leg times the public API with host buffers (
 
   python bench.py --gpus N --steps K --warmup W [--config 2|3|4|5]   # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K ...            # CPU arm: the oracle port of the same path on host cores
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # also write the last timed step's outputs as DIR/<name>.npy
 
 --config selects BASELINE.json `configs[i-1]`: 2 = 4096 Panda Lift OSC_POSE (the headline metric, default), 3 = 8192 Sawyer
 Stack JOINT_VELOCITY, 4 = 16384 Panda NutAssemblyRound, 5 = mixed Lift/Stack/Door/PickPlace, 8192 per GPU (65536 on 8 GPUs)
@@ -253,6 +254,24 @@ def device_timeline(part, groups):
         return None
 
 
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(directory, arrays):
+    """arrays {name: [rows, ...] ndarray} -> directory/<name>.npy in float32 / float64.  Above DUMP_LIMIT_BYTES in all, every
+    array keeps the same fraction of its rows, chosen by a fixed seed, so that two builds dump the same environments."""
+    import numpy as np
+
+    arrays = {k: np.asarray(v, dtype=np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES:
+            keep = max(1, int(a.shape[0] * DUMP_LIMIT_BYTES / total))
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_gpu(args):
     import torch
     import torch.distributed as dist
@@ -346,6 +365,12 @@ def run_gpu(args):
         ev[i][1].record()
     barrier()
     t_wall1 = time.time()
+    # what the last timed step left for its caller, copied before the e2e loop below steps the same environments again
+    outputs = {}
+    if args.dump_outputs and rank == 0:
+        for (task, robot, _, _), e in zip(parts, envs):
+            for k in ("qpos", "qvel", "qacc", "ctrl", "obs", "task_out"):
+                outputs[f"{task}_{robot}_{k}"] = getattr(e.sim, k).cpu().numpy()
     launches = sum(e.sim.launch_count for e in envs) - l0
     ms = sum(a.elapsed_time(b) for a, b in ev)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
@@ -413,6 +438,9 @@ def run_gpu(args):
     e1.record()
     barrier()
     ms2 = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        outputs["e2e_obs"], outputs["e2e_reward"] = h_obs.numpy().copy(), h_rew.numpy().copy()
+        dump_outputs(args.dump_outputs, outputs)
     t2 = torch.tensor([ms2], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t2, op=dist.ReduceOp.MAX)
@@ -541,7 +569,11 @@ def main():
     ap.add_argument("--preroll", type=int, default=100, help="untimed control steps before the timed region")
     ap.add_argument("--mode", type=int, default=int(os.environ.get("B2S_BENCH_MODE", "1")), help="0 fused kernel, 1 phase-kernel pipeline, 2 unit queue (persistent kernel)")
     ap.add_argument("--allgather-obs", type=int, default=1, help="N>1: all-gather observations over NCCL every e2e step")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (rank 0: per task qpos, qvel, qacc, "
+                    "ctrl, obs, task_out; the e2e loop's obs and reward) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs is available for the GPU arm only")
     if args.warmup < 3 and args.impl != "reference":
         args.warmup = 3
     if args.impl == "reference":

@@ -100,82 +100,6 @@ def test_env_api_matches_reference_stack(task):
     env.close()
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/robosuite"), reason="needs the reference checkout (build container only)")
-def test_reference_stack_runs_on_the_shim_and_reproduces_the_golden_file():
-    """regenerate the first two Lift steps with the unmodified reference stack on oracle/mujoco_shim (subprocess: the shim
-    shadows the `mujoco` module name) and compare with the committed vectors"""
-    import subprocess
-    import sys
-
-    code = (
-        "import sys, numpy as np\n"
-        f"sys.path.insert(0, {os.path.join(ROOT, 'tools')!r})\n"
-        "import gen_env_golden as g\n"
-        "g.install()\n"
-        "rec = g.run('Lift', 'Panda', steps=2)\n"
-        "np.save(sys.argv[1], np.concatenate([rec['qpos'].ravel(), rec['obs_object'].ravel(), rec['reward'].ravel()]))\n")
-    out = os.path.join(ROOT, "tests", "golden", "_regen_check.npy")
-    try:
-        r = subprocess.run([sys.executable, "-c", code, out], capture_output=True, text=True, timeout=600)
-        assert r.returncode == 0, r.stderr[-2000:]
-        got = np.load(out)
-    finally:
-        if os.path.exists(out):
-            os.remove(out)
-    G = _golden()
-    ref = np.concatenate([G["Lift/qpos"][:2].ravel(), G["Lift/obs_object"][:2].ravel(), G["Lift/reward"][:2].ravel()])
-    assert np.abs(got - ref).max() < 1e-12
-
-
-@pytest.mark.skipif(not os.path.isdir("/root/reference/robosuite"), reason="needs the reference checkout (build container only)")
-def test_reference_datacollection_episode_loads_and_replays_on_the_oracle(tmp_path):
-    """an episode folder written by the reference's own DataCollectionWrapper (running on the shim) is read by
-    robosuite_b200.state_io; its model.xml compiles, its state rows decode, and replaying the recorded actions from the first
-    state follows the recorded trajectory.  (Not bit-exact by construction: the wrapper re-creates the controllers in
-    reset_from_xml_string BEFORE it restores the recorded state, data_collection_wrapper.py:88-93, so the reference's
-    nullspace posture target differs from the first recorded joint pose; the files do not carry controller state.)"""
-    import subprocess
-    import sys
-
-    code = (
-        "import sys, numpy as np\n"
-        f"sys.path.insert(0, {os.path.join(ROOT, 'tools')!r})\n"
-        "import gen_env_golden as g\n"
-        "g.install()\n"
-        "import robosuite as suite\n"
-        "from robosuite.wrappers import DataCollectionWrapper\n"
-        "env = suite.make('Lift', robots='Panda', has_renderer=False, has_offscreen_renderer=False, use_camera_obs=False,\n"
-        "                 hard_reset=False, control_freq=20, seed=0)\n"
-        "env = DataCollectionWrapper(env, sys.argv[1], collect_freq=1, flush_freq=100)\n"
-        "env.reset()\n"
-        "rng = np.random.default_rng(0)\n"
-        "low, high = env.action_spec\n"
-        "for t in range(4):\n"
-        "    env.step(rng.uniform(low, high))\n"
-        "env.close()\n")
-    r = subprocess.run([sys.executable, "-c", code, str(tmp_path)], capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stderr[-3000:]
-    from oracle.pyoracle import CtrlCfg as OCfg
-    from oracle.pyoracle import Oracle
-    from robosuite_b200 import controller_config as cc
-    from robosuite_b200 import state_io as sio
-    from robosuite_b200.mjcf.compiler import compile_mjcf, pack_model
-
-    eps = [os.path.join(str(tmp_path), d) for d in os.listdir(str(tmp_path)) if d.startswith("ep_")]
-    assert len(eps) == 1
-    ep = sio.load_episode(eps[0])
-    assert ep["env"] == "Lift" and ep["states"].shape[0] == 5 and ep["actions"].shape == (4, 7)
-    m = compile_mjcf(ep["model_xml"])
-    t, q, v = sio.unflatten_state(ep["states"], m.nq, m.nv)
-    o = Oracle(pack_model(m))
-    o.ctrl_setup(cc.resolve(m, cc.default_composite_config(), OCfg))
-    o.qpos[:] = q[0]; o.qvel[:] = v[0]; o.forward(); o.ctrl_reset()
-    assert np.allclose(np.diff(t), 0.05, atol=1e-9) and np.allclose(np.linalg.norm(q[:, -4:], axis=1), 1.0, atol=1e-9)
-    for k in range(4):
-        o.env_step(ep["actions"][k], 25)
-        assert np.abs(o.qpos - q[k + 1]).max() < 3e-2, (k, np.abs(o.qpos - q[k + 1]).max())
-
-
 CPU_CASES = TASKS + ["Lift_JOINT_POSITION", "Lift_JOINT_TORQUE", "Lift_OSC_POSITION", "Lift_Sawyer", "Stack_Sawyer"]
 
 

@@ -1,7 +1,5 @@
-"""tools/compare_with_mujoco.py: the direct oracle-vs-MuJoCo check (VERDICT r1 item 7).  Real MuJoCo is not installable in the build
-container or on the GPU box, so the real comparison skips itself there; the script's plumbing (MJCF rewrite, constant comparison,
-state / control script, gating) is exercised against `oracle/mujoco_shim` (the oracle behind mujoco's API), where every difference
-must be exactly zero."""
+"""tools/compare_with_mujoco.py: the direct oracle-vs-MuJoCo check.  The real comparison needs the `mujoco` package and robosuite's
+mesh files and skips itself where they are absent; the script's seeded state, torque script and MJCF rewrite are checked without them."""
 import importlib
 import os
 import sys
@@ -11,7 +9,6 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-REF_ASSETS = "/root/reference/robosuite/models/assets"
 
 
 def _tool():
@@ -52,23 +49,6 @@ def _real_mujoco():
             sys.modules["mujoco"] = saved
         else:
             sys.modules.pop("mujoco", None)
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_ASSETS), reason="needs the mesh files of the reference checkout (build container only)")
-def test_tool_plumbing_against_the_shim_is_exactly_zero(monkeypatch, capsys):
-    shim = os.path.join(ROOT, "oracle", "mujoco_shim")
-    monkeypatch.syspath_prepend(shim)
-    monkeypatch.delitem(sys.modules, "mujoco", raising=False)
-    t = _tool()
-    rc = t.main(["--assets", REF_ASSETS, "--tasks", "Lift_Panda", "--steps", "30", "--gate-steps", "30"])
-    out = capsys.readouterr().out
-    sys.modules.pop("mujoco", None)
-    assert rc == 0, out
-    import json
-
-    r = json.loads(out)["results"][0]
-    assert r["ok"] and r["gate"]["max_dq_oracle"] == 0.0 and r["gate"]["max_dv_oracle"] == 0.0
-    assert all(v == 0.0 for k, v in r["constants_max_abs_diff"].items() if isinstance(v, float))
 
 
 def test_against_real_mujoco(capsys):
